@@ -5,6 +5,8 @@ nvcc), importing the compute paths raises.
 """
 import ctypes as C
 import os
+import shutil
+import tempfile
 
 from . import build as _build
 
@@ -125,10 +127,13 @@ def lib():
     global _lib
     if _lib is None:
         debug = os.environ.get("OTH_B200_DEBUG", "") not in ("", "0")  # the -DOTH_DEBUG build (arena index assertions)
-        path = _build.LIB_DEBUG if debug else _build.LIB
-        if _build.needs_build(debug):
-            path = _build.build(debug=debug)
+        path, tmp = (_build.LIB_DEBUG if debug else _build.LIB), None
+        if _build.needs_build(debug):  # not what build() left for these sources: compile a private copy, not into the tree
+            tmp = tempfile.mkdtemp(prefix="othello_b200-")
+            path = _build.build(debug=debug, out_dir=tmp)
         L = C.CDLL(path)
+        if tmp:
+            shutil.rmtree(tmp)  # the loaded library stays mapped
         for name, (res, args) in _SIGS.items():
             fn = getattr(L, name)  # AttributeError = ABI mismatch: fail loudly
             fn.restype = res

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MCTS self-play throughput of the B200 engine (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3|c2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3|c2] [--impl reference] [--dump-outputs DIR]
 
 A "step" = `iters_per_step` (= num_simulations) engine iterations: one policy/value forward
 over the leaf batch of every concurrent game + one launch of the fused MCTS kernel, i.e.
@@ -256,6 +256,26 @@ class ClockSampler:
         pw = [float(r[2]) for r in self.rows if len(r) > 2 and r[2].replace(".", "", 1).isdigit()]
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": reasons}
+
+
+DUMP_LIMIT = 64 * 10**6
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT):
+    """Write every float array of ``arrays`` as ``path/<name>.npy``.  If together they would exceed ``limit`` bytes, every
+    array keeps the same fraction of its rows, a sample drawn with a fixed seed from its row count (the kept row indices
+    go to ``<name>_rows.npy``), so that two runs with the same arguments write the same rows."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    limit -= 2 * 128 * len(arrays)  # .npy headers of the data and row-index files
+    need = sum(v.nbytes + 8 * len(v) for v in arrays.values())
+    for name, v in arrays.items():
+        assert v.dtype in (np.float32, np.float64), name
+        if need > limit and len(v):
+            rows = np.sort(np.random.default_rng(0).choice(len(v), max(1, len(v) * limit // need), replace=False))
+            np.save(os.path.join(path, f"{name}_rows.npy"), rows.astype(np.float64))
+            v = v[rows]
+        np.save(os.path.join(path, f"{name}.npy"), v)
 
 
 def measured_peaks():
@@ -560,6 +580,14 @@ def run_b200(a):
     io["h2d"] = io["d2h"] = 0
     ms2, d2 = timed(e2e_step, a.steps)
     e2e_value = total(d2["sims"]) / (ms2 * 1e-3)
+    if a.dump_outputs and rank == 0:
+        # what the last timed step handed to the host for every game: root visit counts (the policy targets) and root value.
+        # The replay tuples of the games that finished in that step are left out: how many finish varies from run to run and
+        # is zero in the opening plies the default window covers.  Two runs of one build differ by a few visits per game:
+        # the de-duplication buckets and the cuDNN plans are chosen by timing, and the network's bf16 results depend on the
+        # batch shape
+        dump_outputs(a.dump_outputs, {"root_visit_counts": pin_counts.numpy().astype(np.float32),
+                                      "root_value": pin_rootv.numpy().copy()})
     if trace:
         print(f"rank {rank} e2e stages (ms):", [(b[0], round((b[1] - a[1]) * 1e3, 1)) for a, b in zip(trace, trace[1:])], file=sys.stderr)
 
@@ -895,6 +923,8 @@ def main():
     ap.add_argument("--dedup", type=int, default=1, help="evaluation de-duplication (oth_mcts_dedup): 1 on (default), 0 off")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-aux", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write every game's root visit counts and root value from the "
+                    "last timed e2e step as DIR/<name>.npy (float32 / float64, at most 64 MB, rank 0)")
     a = ap.parse_args()
     # stdout carries exactly ONE JSON line: everything else this process, its libraries (NCCL prints its
     # version banner to stdout when NCCL_DEBUG is set) and its children write goes to stderr
@@ -917,7 +947,7 @@ def main():
             ref_kind = "reference"
         else:  # no staged reference on this box: the oracle port (C tree/env + the same torch net at batch 1)
             import oracle
-            oracle.build()
+            oracle.lib()
             rate, ms_step, wall = cpu_port_rate(kind, sims, a.steps, a.warmup, cores)
             sample = f"per step every core runs one policy_improve_step of {sims} simulations from the initial position " \
                      f"(batch-1 torch CPU forward per simulation), {cores} processes"
@@ -956,13 +986,13 @@ def main():
             if out["engine"]["evaluation_dedup"]["enabled"]:  # the same plies with every leaf evaluated in its own row
                 out["aux"]["without_dedup"] = aux_selfplay_rate(dev, a.workload, steps=a.steps, warm=a.warmup, dedup=False)
             import oracle
-            oracle.build()
+            oracle.lib()
             rate, games = cpu_env_rate(cores)
             out["aux"]["cpu_env_baseline"] = {"value": rate, "unit": "env steps/s", "cores": cores, "kind": "port",
                                               "sample": f"{games} random playouts (oracle Game-API loop on int8[8,8] boards), {cores} processes x 2 s"}
         if world == 1 and not a.no_cpu_baseline:
             import oracle
-            oracle.build()
+            oracle.lib()
             rate, ms_step, wall = cpu_port_rate(kind, sims, 2, 1, cores)
             port = {"value": rate, "unit": "sims/s", "cores": cores, "kind": "port",
                     "sample": f"{cores} processes x 2 searches of {sims} simulations from the initial position "
@@ -978,5 +1008,15 @@ def main():
         print(json.dumps(out), file=result_out, flush=True)
 
 
+def stop_resource_tracker():
+    """The spawn pools of the CPU arms start multiprocessing's resource tracker, which would outlive this process (and
+    be left to whatever adopts orphans); stop it and reap it here, so the benchmark leaves no process behind."""
+    from multiprocessing import resource_tracker
+    resource_tracker._resource_tracker._stop()
+
+
 if __name__ == "__main__":
-    main()
+    try:
+        main()
+    finally:
+        stop_resource_tracker()

@@ -13,7 +13,9 @@ Parity is pinned by ``tests/test_oracle_golden.py`` against
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -25,12 +27,17 @@ EVAL_FN = C.CFUNCTYPE(None, C.c_void_p, C.POINTER(C.c_int8), C.c_int, C.POINTER(
 STUB_A, STUB_B, STUB_H, STUB_TABLE, STUB_TAPE = 0, 1, 2, 3, 4
 
 
-def build(force=False):
-    """Compile liboracle.so with gcc (oracle/Makefile)."""
-    src = os.path.join(_HERE, "othello_oracle.c")
-    if force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "-B", "liboracle.so"])
-    return _LIB_PATH
+def _stale():
+    return not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(os.path.join(_HERE, "othello_oracle.c"))
+
+
+def build(force=False, out_dir=_HERE):
+    """Compile liboracle.so with gcc (oracle/Makefile) into ``out_dir``; in this directory only when missing or stale,
+    unless ``force``."""
+    lib = os.path.join(out_dir, "liboracle.so")
+    if force or out_dir != _HERE or _stale():
+        subprocess.check_call(["make", "-s", "-C", _HERE, "-B", "OUT=" + lib, lib])
+    return lib
 
 
 _lib = None
@@ -39,8 +46,13 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_LIB_PATH)
+        path, tmp = _LIB_PATH, None
+        if _stale():  # compiled at run time into a temporary directory, never into the tree
+            tmp = tempfile.mkdtemp(prefix="oracle-")
+            path = build(out_dir=tmp)
+        L = C.CDLL(path)
+        if tmp:
+            shutil.rmtree(tmp)  # the loaded library stays mapped
         vp, i32, f64 = C.c_void_p, C.c_int, C.c_double
         L.orc_initial_state.argtypes = [vp]
         L.orc_valid_moves.argtypes = [vp, i32, vp]

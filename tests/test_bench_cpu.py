@@ -22,6 +22,29 @@ def test_workload_config_is_shared_between_the_arms():
     assert set(bench.REF_PLIES_PER_STEP) == set(bench.WORKLOADS)
 
 
+def test_dump_outputs_stays_under_the_limit_with_a_repeatable_sample(tmp_path):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    arrays = {"pis": np.arange(650 * 65, dtype=np.float32).reshape(650, 65), "values": np.arange(650, dtype=np.float64)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    assert sorted(os.listdir(tmp_path / "all")) == ["pis.npy", "values.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "pis.npy"), arrays["pis"])
+    limit = 40000
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, limit=limit)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["pis.npy", "pis_rows.npy", "values.npy", "values_rows.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= limit
+    for f in files:
+        x = np.load(tmp_path / "a" / f)
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, np.load(tmp_path / "b" / f))
+    rows = np.load(tmp_path / "a" / "pis_rows.npy").astype(np.int64)
+    assert len(rows) > 0 and np.array_equal(rows, np.load(tmp_path / "a" / "values_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "pis.npy"), arrays["pis"][rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "values.npy"), arrays["values"][rows])
+
+
 @pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "baseline", "_ref", "self_play_worker.py")),
                     reason="reference not staged (tools/stage_reference.sh)")
 def test_reference_arm_runs_the_staged_reference():
