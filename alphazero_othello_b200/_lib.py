@@ -18,6 +18,7 @@ OTH_MAX_CHILDREN = 40
 
 OTH_OK, OTH_E_CUDA, OTH_E_ARG, OTH_E_ILLEGAL, OTH_E_NO_DEVICE = 0, -1, -2, -3, -4
 F_ILLEGAL, F_TERMINAL, F_WIN, F_LOSS, F_MUST_PASS = 1, 2, 4, 8, 16
+AB_NONE, AB_WIN_SCALE, AB_MAX_DEPTH, AB_MAX_EXACT = -2**31, 10000, 7, 11
 
 EVAL_EXTERNAL, EVAL_STUB_A, EVAL_STUB_B, EVAL_STUB_H, EVAL_ROLLOUT = 0, 1, 2, 3, 4
 PH_RUN, PH_WAIT_EVAL, PH_IDLE, PH_DONE, PH_ERROR, PH_MOVE = 0, 1, 2, 3, 4, 5
@@ -117,6 +118,8 @@ _SIGS = {
     "oth_replay_aggregate": (C.c_int, [C.c_void_p] * 4 + [C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 7),
     "oth_nn_stem_im2col_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "oth_nn_bias_add_relu_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "oth_alphabeta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 4),
+    "oth_host_alphabeta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 3),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGS)

@@ -11,7 +11,8 @@ use one logged uniform per match and ply (``np.random.random_sample``), so a mat
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, alphabeta
+from .alphabeta import AlphaBetaPlayer
 from .engine import MctsEngine, private_copy
 from .envs.othello import OthelloGameNew
 
@@ -74,20 +75,50 @@ class _Side:
                     self.record(self)  # test hook: sees (nn_input, priors, values, phases) of this evaluation
             e.step()
         assert e.counters()["active"] == 0, "search did not finish"
+        self.counts = e.root_stats()["counts"].cpu().numpy()
+
+    def pick(self, i, u):
+        counts = self.counts[i].astype(np.float32)
+        return alphabeta.tie_pick(np.where(counts == counts.max())[0], u)  # MCTS_model.py:249-255, then np.argmax (eval.py:161)
+
+
+class _AlphaBetaSide:
+    """An AlphaBetaPlayer in the arena: one oth_alphabeta launch over the matches it moves in; it keeps no tree."""
+
+    def __init__(self, player, n, device):
+        self.player, self.device = player, device
+        self.has_tree = np.zeros(n, bool)  # never advanced
+        self.values = np.full((n, 65), alphabeta.NONE, np.int32)
+
+    def search(self, mask_np, states, players, sims):
+        idx = np.nonzero(mask_np)[0]
+        own, opp = _pack(states[idx], players[idx])
+        p = self.player
+        values, _, _ = alphabeta.search(torch.from_numpy(own).to(self.device), torch.from_numpy(opp).to(self.device),
+                                        p.depth, p.exact_empties)
+        self.values[idx] = values.cpu().numpy()
+
+    def pick(self, i, u):
+        return alphabeta.pick(self.values[i], self.player.margin, u)
+
+
+def _side(policy, args, n, device, lanes, dtype):
+    return _AlphaBetaSide(policy, n, device) if isinstance(policy, AlphaBetaPlayer) else _Side(policy, args, n, device, lanes, dtype)
 
 
 def play_matches_batched(policy_a, policy_b, args, n_matches, *, device="cuda:0", lanes=None, dtype=torch.bfloat16, record=None,
                          max_plies=128, u_tie=None):
     """n_matches concurrent games; match i: policy_a plays +1 if i is even, policy_b otherwise
-    (eval.py:115-126).  Returns (results, log): results[i] in {"A", "B", "Draw"} from policy_a's
+    (eval.py:115-126).  Either policy, or both, may be a network, a ``DeviceStubPolicy`` or an ``AlphaBetaPlayer``.
+    Returns (results, log): results[i] in {"A", "B", "Draw"} from policy_a's
     point of view as evaluate_models_parallel counts them; log holds per-match actions and tie uniforms.
     ``u_tie`` float64 [n_matches, max_plies]: the tie-pick uniforms to use instead of drawing them (replay of a
     logged match, or of a match of the reference whose np.random.choice(best_actions) picks were tapped)."""
     env = OthelloGameNew(8)
     n = int(n_matches)
     sims = int(args["num_simulations"])
-    A = _Side(policy_a, args, n, device, lanes, dtype)
-    B = _Side(policy_b, args, n, device, lanes, dtype)
+    A = _side(policy_a, args, n, device, lanes, dtype)
+    B = _side(policy_b, args, n, device, lanes, dtype)
     A.record = B.record = record
     a_first = (np.arange(n) % 2 == 0)
     states = np.repeat(env.get_initial_state()[None], n, 0)
@@ -104,14 +135,10 @@ def play_matches_batched(policy_a, policy_b, args, n_matches, *, device="cuda:0"
             A.search(a_moves, states, players, sims)
         if b_moves.any():
             B.search(b_moves, states, players, sims)
-        ca = A.eng.root_stats()["counts"].cpu().numpy()
-        cb = B.eng.root_stats()["counts"].cpu().numpy()
         actions = np.full(n, -1, np.int32)
         for i in np.nonzero(active)[0]:
-            counts = (ca if a_moves[i] else cb)[i].astype(np.float32)
-            best = np.where(counts == counts.max())[0]  # MCTS_model.py:249-255, then np.argmax (eval.py:161)
             u = np.random.random_sample() if u_tie is None else float(u_tie[i, ply])
-            actions[i] = best[min(int(u * len(best)), len(best) - 1)]
+            actions[i] = (A if a_moves[i] else B).pick(i, u)
             log["u_tie"][i, ply] = u
             log["actions"][i, ply] = actions[i]
         idx = np.nonzero(active)[0]
@@ -148,3 +175,12 @@ def evaluate_models_parallel(board_size, args, policy_state, best_policy_state, 
         nets.append(net.eval())
     results, _ = play_matches_batched(nets[0], nets[1], args, n_matches, **kw)
     return results.count("A") / n_matches, results.count("B") / n_matches
+
+
+def evaluate_vs_alphabeta(policy, args, n_matches, player=AlphaBetaPlayer(), **kw):
+    """A network's strength on a fixed scale: ``n_matches`` arena matches of ``policy`` (MCTS with ``args``) against
+    an ``AlphaBetaPlayer``, colours alternating.  Returns ({"win", "draw", "loss"} rates of the network, the match
+    log of ``play_matches_batched``)."""
+    results, log = play_matches_batched(policy, player, args, n_matches, **kw)
+    n = int(n_matches)
+    return {"win": results.count("A") / n, "draw": results.count("Draw") / n, "loss": results.count("B") / n}, log

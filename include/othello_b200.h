@@ -109,7 +109,42 @@ int oth_host_rollout(uint64_t seed, uint64_t game_id_base, int64_t n_games, int3
                      uint64_t* out_final, int64_t n_trace, uint8_t* trace_actions, uint64_t* trace_moves,
                      unsigned long long* total_plies, float* kernel_ms);
 
-/* INT32-ALU roofline probe: dependent-free LOP3/IADD3/SHF mix; returns the
+/* ------------------------------------------------------- alpha-beta player -- */
+
+/* A fixed-depth alpha-beta player: an absolute yardstick for the arena (eval.evaluate_vs_alphabeta).
+ *
+ * For each position (own, opp; own to move) and each legal root action a (board moves, or the pass when the
+ * mover has none), out_values[i][a] = the negamax value of the position after a, from the root mover's side;
+ * every other entry is OTH_AB_NONE.  out_best[i] = the LOWEST action whose value is the maximum, -1 when the
+ * root is terminal.  out_nodes[i][a] (may be NULL) = positions visited below action a (0 if not legal).
+ *
+ * Search semantics (the values are unique: any correct negamax gives them, in any order, with any pruning):
+ *  - every ply costs one depth level; a forced pass is a ply;
+ *  - a position where neither side can move is terminal: OTH_AB_WIN_SCALE * (own discs - opp discs), empty
+ *    squares not awarded (get_score);
+ *  - at depth 0 a non-terminal position scores, from the side to move,
+ *      h = sum_sq W[sq] * (own_sq - opp_sq) + 10 * (#legal(own, opp) - #legal(opp, own)),
+ *    W the D4-symmetric square table, rows 0-3 (rows 4-7 mirror them):
+ *      100 -20  10   5   5  10 -20 100
+ *      -20 -50  -2  -2  -2  -2 -50 -20
+ *       10  -2  -1  -1  -1  -1  -2  10
+ *        5  -2  -1  -1  -1  -1  -2   5
+ *    |h| < 1 300, below one disc of a decided game; all arithmetic is int32;
+ *  - a root with <= exact_empties empty squares is searched to the end of the game (no depth limit).
+ * depth 1..OTH_AB_MAX_DEPTH, exact_empties 0..OTH_AB_MAX_EXACT, else OTH_E_ARG (checked before any device
+ * call).  The caps bound every launch: 4 096 mid-game positions at depth 7 take 1.9 s on a B200 (1 000 W),
+ * 4 096 exact endgames with 11 empties 0.5 s; depth 8 took 16.6 s and 12 empties 3.0 s (DESIGN.md 4). */
+#define OTH_AB_NONE INT32_MIN
+#define OTH_AB_WIN_SCALE 10000
+#define OTH_AB_MAX_DEPTH 7
+#define OTH_AB_MAX_EXACT 11
+int oth_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t depth, int32_t exact_empties,
+                  int32_t* out_values /* [n][65] */, int32_t* out_best /* [n] */, uint64_t* out_nodes /* [n][65] */,
+                  void* stream);
+int oth_host_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t depth, int32_t exact_empties,
+                       int32_t* out_values, int32_t* out_best, uint64_t* out_nodes);
+
+/* INT32-ALU roofline probe:dependent-free LOP3/IADD3/SHF mix; returns the
  * measured thread-instructions per second in *out_ips (BASELINE.md 3). */
 int oth_host_int32_peak(double* out_ips, float* kernel_ms);
 
