@@ -1,10 +1,14 @@
 // Batched fixed-depth alpha-beta player (oth_alphabeta): a fixed yardstick opponent for the arena.
 //
-// One warp per position; lane l searches the root actions of rank l, l+32 (ascending action order) with a
-// full-window alpha-beta below each of them, so every root value is the exact negamax value whatever the
-// move ordering inside a subtree.  The search semantics (ply = one depth level, forced pass included,
-// terminal = 10 000 x disc difference, depth-0 heuristic) are defined once, in ab_leaf() / ab_subtree() below,
-// and documented in include/othello_b200.h; tests/alphabeta_oracle.c restates them on the CPU oracle's mailbox boards.
+// One warp per position, two kernels that split the roots of a launch between them:
+//  - k_alphabeta (depth-limited roots, and exact ones with <= 11 empties): lane l searches the root actions of rank l,
+//    l+32 (ascending action order) with a full-window alpha-beta below each of them;
+//  - k_alphabeta_split (exact roots with 12 or more empties): the Young Brothers Wait split one level below each root
+//    action, so the warp's lanes share (root action, reply) tasks instead of idling beside the longest root action.
+// Either way every root value is the exact negamax value whatever the move ordering inside a subtree.  The search
+// semantics (ply = one depth level, forced pass included, terminal = 10 000 x disc difference, depth-0 heuristic) are
+// defined once, in ab_leaf() / ab_subtree() below, and documented in include/othello_b200.h;
+// tests/alphabeta_oracle.c restates them on the CPU oracle's mailbox boards.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -21,6 +25,8 @@ namespace {
 // at most OTH_AB_MAX_DEPTH - 1.
 constexpr int AB_STACK = 2 * OTH_AB_MAX_EXACT + 2;
 static_assert(AB_STACK >= OTH_AB_MAX_DEPTH, "stack shorter than the depth cap");
+// The most empties k_alphabeta solves exactly.  Its roots keep their values and node counts whatever the cap above.
+constexpr int AB_SEQ_MAX_EXACT = 11;
 constexpr int AB_INF = 1 << 30;   // > every value: |terminal| <= 640 000, |heuristic| < 1 300
 constexpr u64 PASS_ONLY = ~0ULL;  // "remaining moves" of a node whose only action is the pass (no real move set is full)
 
@@ -88,12 +94,12 @@ struct Frame {
     int alpha, beta;
 };
 
-// Exact negamax value of (own, opp) searched `depth` plies deep: iterative fail-hard alpha-beta with a full
-// window at the top.  *nodes += positions visited.
-__device__ int ab_subtree(u64 own, u64 opp, int depth, unsigned long long* nodes)
+// Negamax value of (own, opp) searched `depth` plies deep: iterative fail-hard alpha-beta with the window
+// (alpha, beta) at the top, exact when it lies inside the window, beta when it is >= beta.  *nodes += positions visited.
+__device__ int ab_subtree(u64 own, u64 opp, int depth, int alpha, int beta, unsigned long long* nodes)
 {
     Frame st[AB_STACK];
-    int sp = 0, alpha = -AB_INF, beta = AB_INF, v;
+    int sp = 0, v;
     u64 rem;
     unsigned long long cnt = 0;
     for (;;) {
@@ -137,6 +143,12 @@ __device__ int ab_subtree(u64 own, u64 opp, int depth, unsigned long long* nodes
     }
 }
 
+// Whether a root is searched by k_alphabeta_split: only the exact searches beyond k_alphabeta's.
+__device__ __forceinline__ bool ab_split_root(int empties, int exact_empties)
+{
+    return empties <= exact_empties && empties > AB_SEQ_MAX_EXACT;
+}
+
 __global__ void __launch_bounds__(128) k_alphabeta(const u64* __restrict__ own_in, const u64* __restrict__ opp_in, int64_t n,
                                                    int depth, int exact_empties, int32_t* __restrict__ out_values,
                                                    int32_t* __restrict__ out_best, unsigned long long* __restrict__ out_nodes)
@@ -148,8 +160,10 @@ __global__ void __launch_bounds__(128) k_alphabeta(const u64* __restrict__ own_i
         const u64 m = legal_moves(own, opp);
         const bool pass = !m && legal_moves(opp, own);
         const int k = m ? __popcll(m) : (pass ? 1 : 0);  // root actions; 0 = terminal root
+        const int empties = 64 - __popcll(own | opp);
+        if (ab_split_root(empties, exact_empties)) continue;  // k_alphabeta_split's root
         // below a root action: depth - 1 plies, or (exact) deeper than any game from here can last
-        const int sub_depth = (64 - __popcll(own | opp) <= exact_empties) ? AB_STACK : depth - 1;
+        const int sub_depth = empties <= exact_empties ? AB_STACK : depth - 1;
         int val[2] = {OTH_AB_NONE, OTH_AB_NONE};
         unsigned long long cnt[2] = {0, 0};
         int best_v = OTH_AB_NONE, best_a = 65;
@@ -159,7 +173,7 @@ __global__ void __launch_bounds__(128) k_alphabeta(const u64* __restrict__ own_i
             if (r < k) {
                 const int a = pass ? OTH_PASS : nth_set_bit(m, r);
                 const Board c = apply_move(own, opp, a, pass ? 0ULL : flips(own, opp, 1ULL << a));
-                val[s] = -ab_subtree(c.own, c.opp, sub_depth, &cnt[s]);
+                val[s] = -ab_subtree(c.own, c.opp, sub_depth, -AB_INF, AB_INF, &cnt[s]);
                 if (val[s] > best_v) {  // ranks ascend with the action index: the first maximum is the lowest action
                     best_v = val[s];
                     best_a = a;
@@ -191,6 +205,119 @@ __global__ void __launch_bounds__(128) k_alphabeta(const u64* __restrict__ own_i
     }
 }
 
+// Per-warp state of one root in k_alphabeta_split, indexed by root-action rank (a position has < 64 actions).
+struct SplitRoot {
+    int next;              // next task to claim
+    int ntasks;
+    int young_begin[65];   // younger-brother tasks of rank r: ntasks' indices k + young_begin[r] .. k + young_begin[r+1]-1
+    u64 young[64];         // their reply squares (the child's actions minus the eldest)
+    int beta[64];          // window top of those tasks = the eldest's value; AB_INF until it is known
+    int val[64];           // min over the rank's task results = its root value
+    unsigned long long nodes[64];
+};
+
+// Exact roots beyond k_alphabeta's (ab_split_root), one warp each, split one level below the root actions
+// (Young Brothers Wait).  For root action a with child c and replies g_1 .. g_m (ab_next_child's order):
+//  - eldest task: g_1 with a full window, so L = -V(g_1) is a lower bound on V(c);
+//  - younger tasks: every other g_j with the window (-AB_INF, -L), fail-hard, so -result = max(L, -V(g_j)) exactly;
+// and the root value -V(c) = min(V(g_1), min_j result_j).  A child that is terminal, a forced pass or has one
+// reply is one task (its whole subtree).  The lanes claim tasks from a counter, eldest tasks first; a younger
+// task waits for its eldest.  Every task's window is fixed by the position alone and results are combined with min
+// and sum, so values and node counts do not depend on which lane ran which task.
+__global__ void __launch_bounds__(128) k_alphabeta_split(const u64* __restrict__ own_in, const u64* __restrict__ opp_in,
+                                                         int64_t n, int exact_empties,
+                                                         int32_t* __restrict__ out_values, int32_t* __restrict__ out_best,
+                                                         unsigned long long* __restrict__ out_nodes)
+{
+    __shared__ SplitRoot sh_roots[4];
+    SplitRoot& R = sh_roots[threadIdx.x >> 5];
+    const int lane = threadIdx.x & 31;
+    const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += nw) {
+        const u64 own = own_in[i], opp = opp_in[i];
+        if (!ab_split_root(64 - __popcll(own | opp), exact_empties)) continue;
+        const u64 m = legal_moves(own, opp);
+        const bool pass = !m && legal_moves(opp, own);
+        const int k = m ? __popcll(m) : (pass ? 1 : 0);
+        // the tasks of every root action
+        for (int r = lane; r < k; r += 32) {
+            const int a = pass ? OTH_PASS : nth_set_bit(m, r);
+            const Board c = apply_move(own, opp, a, pass ? 0ULL : flips(own, opp, 1ULL << a));
+            int v;
+            u64 rem = 0;
+            if (!ab_leaf(c.own, c.opp, AB_STACK, &v, &rem) && rem != PASS_ONLY)
+                ab_next_child(c.own, c.opp, &rem);  // rem = the younger brothers
+            else
+                rem = 0;
+            R.young[r] = rem;
+            R.young_begin[r + 1] = __popcll(rem);
+            R.beta[r] = AB_INF;
+            R.val[r] = AB_INF;
+            R.nodes[r] = 0;
+        }
+        __syncwarp();
+        if (lane == 0) {
+            R.young_begin[0] = 0;
+            for (int r = 0; r < k; r++) R.young_begin[r + 1] += R.young_begin[r];
+            R.ntasks = k + R.young_begin[k];
+            R.next = 0;
+        }
+        __syncwarp();
+        for (int t = atomicAdd(&R.next, 1); t < R.ntasks; t = atomicAdd(&R.next, 1)) {
+            int r = t;
+            if (t >= k)
+                for (r = 0; t - k >= R.young_begin[r + 1]; r++) {}
+            const int a = pass ? OTH_PASS : nth_set_bit(m, r);
+            const Board c = apply_move(own, opp, a, pass ? 0ULL : flips(own, opp, 1ULL << a));
+            unsigned long long cnt = 0;
+            int v;
+            if (t >= k) {  // younger brother: wait for the eldest's value
+                volatile int* vb = &R.beta[r];
+                int beta;
+                while ((beta = *vb) == AB_INF) __nanosleep(256);
+                const int sq = nth_set_bit(R.young[r], t - k - R.young_begin[r]);
+                const Board g = apply_move(c.own, c.opp, sq, flips(c.own, c.opp, 1ULL << sq));
+                v = ab_subtree(g.own, g.opp, AB_STACK - 1, -AB_INF, beta, &cnt);
+            } else if (R.young[r]) {  // eldest brother
+                u64 rem = legal_moves(c.own, c.opp);
+                const Board g = ab_next_child(c.own, c.opp, &rem);
+                v = ab_subtree(g.own, g.opp, AB_STACK - 1, -AB_INF, AB_INF, &cnt);
+                cnt++;  // c
+                *(volatile int*)&R.beta[r] = v;
+            } else {  // c unsplit
+                v = -ab_subtree(c.own, c.opp, AB_STACK, -AB_INF, AB_INF, &cnt);
+            }
+            atomicMin(&R.val[r], v);
+            atomicAdd(&R.nodes[r], cnt);
+        }
+        __syncwarp();
+        // lowest action among the maxima, as in k_alphabeta
+        int best_v = OTH_AB_NONE, best_a = 65;
+        for (int r = lane; r < k; r += 32) {
+            const int a = pass ? OTH_PASS : nth_set_bit(m, r);
+            if (R.val[r] > best_v || (R.val[r] == best_v && a < best_a)) {
+                best_v = R.val[r];
+                best_a = a;
+            }
+        }
+        for (int o = 16; o; o >>= 1) {
+            const int ov = __shfl_xor_sync(0xffffffffu, best_v, o), oa = __shfl_xor_sync(0xffffffffu, best_a, o);
+            if (ov > best_v || (ov == best_v && oa < best_a)) {
+                best_v = ov;
+                best_a = oa;
+            }
+        }
+        if (lane == 0) out_best[i] = k ? best_a : -1;
+        for (int e = lane; e < OTH_NUM_ACTIONS; e += 32) {
+            const bool legal = e < 64 ? ((m >> e) & 1) : pass;
+            const int r = e < 64 ? __popcll(m & ((1ULL << e) - 1)) : 0;
+            out_values[i * OTH_NUM_ACTIONS + e] = legal ? R.val[r] : OTH_AB_NONE;
+            if (out_nodes) out_nodes[i * OTH_NUM_ACTIONS + e] = legal ? R.nodes[r] : 0ULL;
+        }
+        __syncwarp();  // R is reused by the warp's next root
+    }
+}
+
 }  // namespace
 
 extern "C" int oth_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t depth, int32_t exact_empties,
@@ -201,7 +328,13 @@ extern "C" int oth_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n
     if (!own || !opp || !out_values || !out_best) return OTH_E_ARG;
     k_alphabeta<<<grid_for(n * 32, 128), 128, 0, (cudaStream_t)stream>>>((const u64*)own, (const u64*)opp, n, depth, exact_empties,
                                                                          out_values, out_best, (unsigned long long*)out_nodes);
-    return cuda_status(cudaGetLastError());
+    int rc = cuda_status(cudaGetLastError());
+    if (rc == OTH_OK && exact_empties > AB_SEQ_MAX_EXACT) {
+        k_alphabeta_split<<<grid_for(n * 32, 128), 128, 0, (cudaStream_t)stream>>>(
+            (const u64*)own, (const u64*)opp, n, exact_empties, out_values, out_best, (unsigned long long*)out_nodes);
+        rc = cuda_status(cudaGetLastError());
+    }
+    return rc;
 }
 
 extern "C" int oth_host_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t depth, int32_t exact_empties,

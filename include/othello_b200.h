@@ -116,7 +116,8 @@ int oth_host_rollout(uint64_t seed, uint64_t game_id_base, int64_t n_games, int3
  * For each position (own, opp; own to move) and each legal root action a (board moves, or the pass when the
  * mover has none), out_values[i][a] = the negamax value of the position after a, from the root mover's side;
  * every other entry is OTH_AB_NONE.  out_best[i] = the LOWEST action whose value is the maximum, -1 when the
- * root is terminal.  out_nodes[i][a] (may be NULL) = positions visited below action a (0 if not legal).
+ * root is terminal.  out_nodes[i][a] (may be NULL) = positions visited below action a, the position after a
+ * included: > 0 exactly for the legal actions.  It depends on how the root is searched (below), not on the launch.
  *
  * Search semantics (the values are unique: any correct negamax gives them, in any order, with any pruning):
  *  - every ply costs one depth level; a forced pass is a ply;
@@ -132,12 +133,20 @@ int oth_host_rollout(uint64_t seed, uint64_t game_id_base, int64_t n_games, int3
  *    |h| < 1 300, below one disc of a decided game; all arithmetic is int32;
  *  - a root with <= exact_empties empty squares is searched to the end of the game (no depth limit).
  * depth 1..OTH_AB_MAX_DEPTH, exact_empties 0..OTH_AB_MAX_EXACT, else OTH_E_ARG (checked before any device
- * call).  The caps bound every launch: 4 096 mid-game positions at depth 7 take 1.9 s on a B200 (1 000 W),
- * 4 096 exact endgames with 11 empties 0.5 s; depth 8 took 16.6 s and 12 empties 3.0 s (DESIGN.md 4). */
+ * call).
+ *
+ * The search, one warp per position: a depth-limited root, or an exact one with <= 11 empties, gives each root
+ * action to one lane, which runs a full-window alpha-beta below it.  An exact root with 12..exact_empties empties is
+ * split one level further (Young Brothers Wait): below root action a, the first reply in the search's move order is
+ * searched with a full window, which bounds the value of the position after a; every other reply is then its own
+ * task, searched with the window that bound leaves (fail-hard), and the warp's lanes share these tasks.  On that
+ * path out_nodes counts the positions of all these searches.  The caps bound every launch: 4 096 mid-game positions
+ * at depth 7 take 1.9 s on a B200 (1 000 W), 4 096 exact endgames with 12 empties 2.0 s.  Depth 8 (11.7 s) and
+ * 13 empties (10.7 s) miss a 4 s budget even on the split search (DESIGN.md 4). */
 #define OTH_AB_NONE INT32_MIN
 #define OTH_AB_WIN_SCALE 10000
 #define OTH_AB_MAX_DEPTH 7
-#define OTH_AB_MAX_EXACT 11
+#define OTH_AB_MAX_EXACT 12
 int oth_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t depth, int32_t exact_empties,
                   int32_t* out_values /* [n][65] */, int32_t* out_best /* [n] */, uint64_t* out_nodes /* [n][65] */,
                   void* stream);

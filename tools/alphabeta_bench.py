@@ -3,11 +3,15 @@
     python tools/alphabeta_bench.py --out profiles/alphabeta_bench.json
 
 - positions/s and nodes/s at depths 2/4/6/7 (mid-game and late-game roots; 7 = OTH_AB_MAX_DEPTH) and exactly solved
-  endgames with 10/11 empties (11 = OTH_AB_MAX_EXACT), over 4 096 and 16 384 roots: CUDA events around whole launches,
-  after one warm-up launch of the same shape;
-- lane balance = sum of nodes / (32 x the largest per-lane node count), summed over warps (one warp per root, lane l
-  searches the root actions of rank l and l + 32): the share of lane-time that does work;
-- wall time of 1 024 arena matches of a FastOthelloNet (100 simulations per move) against depth 4 and depth 6.
+  endgames with 10/11/12 empties (12 = OTH_AB_MAX_EXACT), over 4 096 and 16 384 roots, and over 512 roots (the batch
+  an arena ply searches) at depth 7 and 11 and 12 exact empties: CUDA events around whole launches, after one warm-up
+  launch of the same shape;
+- lane balance, for the roots k_alphabeta searches (all but exact ones with 12+ empties) = sum of nodes / (32 x the
+  largest per-lane node count), summed over warps (one warp per root, lane l searches the root actions of rank l and
+  l + 32): the share of lane-time that does work.  The split search's lanes share (root action, reply) tasks
+  dynamically, so no formula gives their lanes; its cases report launch time, nodes/s and nodes per position;
+- wall time of 1 024 arena matches of a FastOthelloNet (100 simulations per move) against depth 4 and depth 6 (exact
+  from 10 empties) and depth 7 (exact from 12 empties).
 Roots come from uniform-random games played by the library's own rollout kernel (seeded).  The GPU's name and power
 limit are read in the same run.
 """
@@ -79,7 +83,7 @@ def lane_balance(values, nodes):
     return float(per_lane.sum() / (32 * per_lane.max(1)).sum())
 
 
-def time_search(own, opp, depth, exact, reps):
+def time_search(own, opp, depth, exact, reps, split):
     search(own, opp, depth, exact)  # warm-up: same shape
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -94,10 +98,12 @@ def time_search(own, opp, depth, exact, reps):
     n = len(v)
     total = int(nodes.sum())
     t = min(ms) / 1e3
-    return {"positions": n, "depth": depth, "exact_empties": exact, "launch_ms": [round(x, 3) for x in ms],
-            "positions_per_s": n / t, "nodes": total, "nodes_per_s": total / t,
-            "nodes_per_position": total / n, "lane_balance": lane_balance(v, nodes),
-            "mean_root_actions": float((v != _lib.AB_NONE).sum(1).mean())}
+    r = {"positions": n, "depth": depth, "exact_empties": exact, "launch_ms": [round(x, 3) for x in ms],
+         "positions_per_s": n / t, "nodes": total, "nodes_per_s": total / t, "nodes_per_position": total / n,
+         "mean_root_actions": float((v != _lib.AB_NONE).sum(1).mean())}
+    if not split:
+        r["lane_balance"] = lane_balance(v, nodes)
+    return r
 
 
 def main():
@@ -107,33 +113,36 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--arena-matches", type=int, default=1024)
     ap.add_argument("--arena-sims", type=int, default=100)
-    ap.add_argument("--arena-depths", default="4,6")
+    ap.add_argument("--arena-levels", default="4:10,6:10,7:12", help="depth:exact_empties of each arena run")
     a = ap.parse_args()
     assert torch.cuda.is_available(), "needs a CUDA device"
     res = {"gpu": gpu_info(), "search": [], "arena": []}
     sizes = [int(x) for x in a.sizes.split(",")]
     cases = [("mid-game", 40, d, 0) for d in (2, 4, 6, 7)] + [("late-game", 24, d, 0) for d in (2, 4, 6, 7)] + \
-            [("endgame", e, 1, e) for e in (10, 11)]
-    for n in sizes:
-        for phase, empties, depth, exact in cases:
-            own, opp = roots(n, empties, seed=1000 + empties)
-            r = time_search(own, opp, depth, exact, a.reps)
-            r.update(phase=phase, root_empties=empties)
-            print(json.dumps(r), flush=True)
-            res["search"].append(r)
+            [("endgame", e, 1, e) for e in (10, 11, 12)]
+    arena_batch = [("mid-game", 40, 7, 0)] + [("endgame", e, 1, e) for e in (11, 12)]
+    for n, case in [(n, c) for n in sizes for c in cases] + [(512, c) for c in arena_batch]:
+        phase, empties, depth, exact = case
+        split = 11 < empties <= exact  # every root of a case has `empties` empty squares: one path searches them all
+        own, opp = roots(n, empties, seed=1000 + empties)
+        r = time_search(own, opp, depth, exact, a.reps, split)
+        r.update(phase=phase, root_empties=empties, path="split" if split else "per-action")
+        print(json.dumps(r), flush=True)
+        res["search"].append(r)
     from alphazero_othello_b200.Models import FastOthelloNet
     from alphazero_othello_b200.eval import evaluate_vs_alphabeta
     torch.manual_seed(0)
     net = FastOthelloNet(8, 65).eval()
     args = {"c_puct": 2.0, "num_simulations": a.arena_sims}
-    for d in [int(x) for x in a.arena_depths.split(",") if x]:
+    for level in [x for x in a.arena_levels.split(",") if x]:
+        d, x = (int(v) for v in level.split(":"))
         np.random.seed(0)
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        rates, log = evaluate_vs_alphabeta(net, args, a.arena_matches, player=AlphaBetaPlayer(depth=d, exact_empties=10))
+        rates, log = evaluate_vs_alphabeta(net, args, a.arena_matches, player=AlphaBetaPlayer(depth=d, exact_empties=x))
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
-        r = {"matches": a.arena_matches, "simulations": a.arena_sims, "depth": d, "exact_empties": 10, "wall_s": dt,
+        r = {"matches": a.arena_matches, "simulations": a.arena_sims, "depth": d, "exact_empties": x, "wall_s": dt,
              "plies": int(log["plies"].sum()), "rates": rates}
         print(json.dumps(r), flush=True)
         res["arena"].append(r)
