@@ -12,7 +12,7 @@
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, endgame
 from .MCTS_model import MCTS
 from .engine import BatchedPolicy, MctsEngine, SelfPlayRunner, private_copy, split_games
 from .envs.othello import OthelloGameNew as OthelloGame
@@ -75,9 +75,13 @@ def one_self_play(args_tuple):
 
 
 def collect_self_play_games(policy, args, n_games, *, n_slots=None, device="cuda:0", dtype=torch.bfloat16, seed=0,
-                            game_id_base=0, fold=True, use_graph=True, return_raw=False, dedup="auto"):
-    """Play ``n_games`` self-play games with ``policy`` (a torch module) on one GPU."""
+                            game_id_base=0, fold=True, use_graph=True, return_raw=False, dedup="auto", solve_empties=0):
+    """Play ``n_games`` self-play games with ``policy`` (a torch module) on one GPU.  With ``solve_empties`` > 0 the
+    value target of every position with at most that many empty squares is its solved win / draw / loss
+    (``endgame.relabel``) instead of its lambda-return."""
     from .Models import fold_for_inference
+    if not 0 <= int(solve_empties) <= endgame.MAX_EMPTIES:
+        raise ValueError(f"solve_empties must be in 0..{endgame.MAX_EMPTIES}, got {solve_empties}")
     n_slots = int(n_slots or min(n_games, 4096))
     gps = -(-n_games // n_slots)
     eng = MctsEngine(n_slots, args, self_play=True, eval_kind=_lib.EVAL_EXTERNAL, games_per_slot=gps, device=device,
@@ -90,6 +94,8 @@ def collect_self_play_games(policy, args, n_games, *, n_slots=None, device="cuda
         ev = BatchedPolicy(net, device, dtype)
     out = SelfPlayRunner(eng, ev, use_graph=use_graph, dedup=dedup).play()
     eng.raise_on_error()
+    if solve_empties:
+        out = endgame.relabel(out, solve_empties, device=device)
     return out if return_raw else split_games(out)[:n_games]
 
 

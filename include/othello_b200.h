@@ -153,6 +153,30 @@ int oth_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t d
 int oth_host_alphabeta(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t depth, int32_t exact_empties,
                        int32_t* out_values, int32_t* out_best, uint64_t* out_nodes);
 
+/* ------------------------------------------------------- endgame solver -- */
+
+/* The game-theoretic result of endgame positions: the truth a self-play value target can be replaced with
+ * (endgame.relabel).
+ *
+ * For each position (own, opp; own to move) with at most max_empties empty squares, out_wld[i] = +1, 0 or -1: the
+ * result for own under perfect play by both sides to the end of the game, forced passes included.  The result is the
+ * sign of the final disc difference, empty squares not awarded (get_value_and_terminated; the sign of oth_alphabeta's
+ * exact values).  A terminal position gets its own result.  A position with more empty squares gets
+ * OTH_WLD_UNSOLVED and 0 nodes.  out_nodes[i] (may be NULL) = positions the search visited, the root included; it
+ * depends on the position alone, not on the launch.  max_empties 0..OTH_SOLVE_MAX_EMPTIES, else OTH_E_ARG (checked
+ * before any device call).
+ *
+ * The search, one thread per position: a sequential alpha-beta with the window (-1, +1) on that sign, which stops at
+ * the first winning move; children are searched fastest-first (fewest replies for the opponent) from 7 empty squares
+ * up, in the alpha-beta player's static order below.  The cap bounds a launch: 4 096 positions with 14 empties took
+ * 1.53 s on a B200 (1 000 W), with 15 empties 7.7 s and with 16 empties 54 s (DESIGN.md 4). */
+#define OTH_SOLVE_MAX_EMPTIES 14
+#define OTH_WLD_UNSOLVED (-128)
+int oth_solve_wld(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t max_empties, int8_t* out_wld /* [n] */,
+                  uint64_t* out_nodes /* [n] */, void* stream);
+int oth_host_solve_wld(const uint64_t* own, const uint64_t* opp, int64_t n, int32_t max_empties, int8_t* out_wld,
+                       uint64_t* out_nodes);
+
 /* INT32-ALU roofline probe:dependent-free LOP3/IADD3/SHF mix; returns the
  * measured thread-instructions per second in *out_ips (BASELINE.md 3). */
 int oth_host_int32_peak(double* out_ips, float* kernel_ms);
