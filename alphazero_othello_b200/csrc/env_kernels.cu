@@ -295,6 +295,10 @@ __global__ void __launch_bounds__(256) k_symmetry(const int8_t* __restrict__ sta
 // Network-boundary epilogue (the network itself stays PyTorch/cuDNN): x = relu(x + bias[c] + res)
 // on channels-last bf16 activations, 8 elements (128 bits) per thread.
 #include <cuda_bf16.h>
+// relu that keeps a NaN, as torch.relu does: fmaxf(NaN, 0) would return 0 and hide it from the non-finite guard;
+// every other input takes the same fmaxf as before, bit for bit
+__device__ __forceinline__ float relu_keep_nan(float v) { return v != v ? v : fmaxf(v, 0.0f); }
+
 __global__ void __launch_bounds__(256) k_bias_add_relu_bf16(uint4* __restrict__ x, const uint4* __restrict__ res,
                                                             const __nv_bfloat16* __restrict__ bias, int64_t n8, int C)
 {
@@ -310,7 +314,7 @@ __global__ void __launch_bounds__(256) k_bias_add_relu_bf16(uint4* __restrict__ 
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             const float2 fa = __bfloat1622float2(pa[k]), fr = __bfloat1622float2(pr[k]), fb = __bfloat1622float2(pb[k]);
-            pa[k] = __floats2bfloat162_rn(fmaxf(fa.x + fb.x + fr.x, 0.0f), fmaxf(fa.y + fb.y + fr.y, 0.0f));
+            pa[k] = __floats2bfloat162_rn(relu_keep_nan(fa.x + fb.x + fr.x), relu_keep_nan(fa.y + fb.y + fr.y));
         }
         x[i] = a;
     }
