@@ -16,6 +16,10 @@ the GPU straight from the engine's leaf batch) or any object with
 leaf, MCTS_model.py:276-303, 332-335) evaluated in-kernel; its playouts draw from the engine's
 Philox streams (keyed by ``seed``), not from ``np.random``.
 
+``leaf_symmetry`` (torch-module policies only): ``"random"`` evaluates every leaf in one of its eight orientations,
+drawn from (``seed``, position), and maps the policy back; ``"mean"`` evaluates all eight and averages priors and
+values (symmetry.py).  ``apply_symmetry``, the reference's dead switch for the same idea, stays accepted and ignored.
+
 Restrictions (stated, not silent): ``args["num_threads"]`` is accepted and ignored -- searches
 run with the reference's ``num_threads=1`` semantics, the only deterministic mode (its default
 of 4 races virtual losses between Python threads); the caller's ``policy`` module is neither
@@ -25,7 +29,7 @@ moved nor switched to eval mode, the search works on a private copy made at cons
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, symmetry
 from .engine import MctsEngine, private_copy
 
 
@@ -53,7 +57,10 @@ class _Root:
 
 class MCTS:
     def __init__(self, env, args, policy, apply_symmetry=False, dirichlet_alpha=0.03, dirichlet_epsilon=0.0,
-                 inference_cache=None, device="cuda:0", seed=0):
+                 inference_cache=None, device="cuda:0", seed=0, leaf_symmetry=None):
+        self.leaf_symmetry = symmetry.check_mode(leaf_symmetry)
+        if self.leaf_symmetry and not isinstance(policy, torch.nn.Module):
+            raise ValueError("leaf_symmetry needs a torch module policy (the network is evaluated on the device)")
         self.env, self.args, self.policy = env, args, policy
         self.use_rollout = policy is None
         self.num_actions = env.action_size
@@ -69,6 +76,12 @@ class MCTS:
         self._module = isinstance(policy, torch.nn.Module)
         if self._module:
             self.policy = private_copy(policy, self.device)
+        self._seed = int(seed)
+        if self.leaf_symmetry == "random":
+            self._xs = torch.zeros_like(self._e.nn_input)
+            self._sym = torch.zeros(1, dtype=torch.uint8, device=self.device)
+        elif self.leaf_symmetry == "mean":
+            self._images = torch.zeros((8, 1, 8, 8), dtype=torch.float32, device=self.device)
         self._graph = None        # CUDA graph of (network forward + oth_mcts_step) for module policies
         self._graph_failed = False
         self._state = None  # host copy of the root position
@@ -93,8 +106,20 @@ class MCTS:
     def _evaluate(self):
         e = self._e
         if self._module:
-            logits, value = self.policy(e.nn_input)
-            e.priors.copy_(torch.softmax(logits.float(), -1))
+            if self.leaf_symmetry == "mean":
+                symmetry.images(e.nn_input, self._images)
+                logits, value = self.policy(self._images)
+                symmetry.mean(logits.float(), value.float().reshape(-1), e.priors, e.values)
+                return
+            x = e.nn_input
+            if self.leaf_symmetry == "random":
+                symmetry.leaf_symmetry(x, self._seed, self._xs, self._sym)
+                x = self._xs
+            logits, value = self.policy(x)
+            logits = logits.float()
+            if self.leaf_symmetry == "random":
+                symmetry.unsymmetrise_logits(logits, self._sym)
+            e.priors.copy_(torch.softmax(logits, -1))
             e.values.copy_(value.float().reshape(-1))
             return
         canon = e.nn_input.view(8, 8).cpu().numpy().astype(np.int8)

@@ -119,6 +119,11 @@ _SIGS = {
     "oth_replay_aggregate": (C.c_int, [C.c_void_p] * 4 + [C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 7),
     "oth_nn_stem_im2col_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "oth_nn_bias_add_relu_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "oth_nn_leaf_symmetry": (C.c_int, [C.c_void_p, C.c_int64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "oth_nn_unsymmetrise_logits": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
+    "oth_nn_symmetry_images": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "oth_nn_symmetry_mean": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
+                                       C.c_void_p]),
     "oth_alphabeta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 4),
     "oth_host_alphabeta": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 3),
     "oth_solve_wld": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32] + [C.c_void_p] * 3),

@@ -17,7 +17,7 @@ INCLUDE = os.path.join(HERE, "..", "include")
 LIB = os.path.join(HERE, "libothello_b200.so")
 LIB_DEBUG = os.path.join(HERE, "libothello_b200_debug.so")  # -DOTH_DEBUG: arena index assertions (OTH_B200_DEBUG=1 loads it)
 SOURCES = ["env_kernels.cu", "mcts_kernels.cu", "replay_kernels.cu", "dedup_kernels.cu", "alphabeta_kernels.cu",
-           "endgame_kernels.cu"]
+           "endgame_kernels.cu", "symmetry_kernels.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

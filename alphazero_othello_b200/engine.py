@@ -12,7 +12,7 @@ import os
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, symmetry
 
 
 def default_lanes(n_slots):
@@ -279,11 +279,15 @@ class BatchedPolicy:
         return self.policy(x, raw=True)
 
     @torch.no_grad()
-    def __call__(self, x, priors_out, values_out):
+    def __call__(self, x, priors_out, values_out, sym=None):
+        """``sym`` (uint8 [B], optional): row i of ``x`` is the leaf in orientation T_sym[i] (symmetry.leaf_symmetry);
+        its logits are mapped back to the leaf's orientation before the softmax."""
         if self.has_raw:
             # network twin: logits / value pre-activation straight from the head GEMMs; one softmax kernel
             # (cast fused) and one cast + one tanh for the values
             logits, v = self.policy(x, raw=True)
+            if sym is not None:
+                symmetry.unsymmetrise_logits(logits, sym)
             torch.softmax(logits, dim=-1, dtype=torch.float32, out=priors_out)
             values_out.copy_(v.reshape(-1))
             values_out.tanh_()
@@ -293,7 +297,10 @@ class BatchedPolicy:
                 logits, value = self.policy(x)
         else:
             logits, value = self.policy(x)
-        torch.softmax(logits.float(), dim=-1, out=priors_out)
+        logits = logits.float()
+        if sym is not None:
+            symmetry.unsymmetrise_logits(logits, sym)
+        torch.softmax(logits, dim=-1, out=priors_out)
         values_out.copy_(value.float().reshape(-1))
 
 
@@ -307,13 +314,21 @@ class SelfPlayRunner:
     slot's outputs through an index map.  The bucket is chosen on the host from the distinct-position count the device
     reported a few iterations earlier; positions that do not fit the bucket just wait one launch, so the choice only
     affects speed.  "auto" enables it for the fused pipeline from 8192 slots up (measured: at 4096 slots of the
-    small network a half-size batch costs 2/3 of a full one and the compaction pass eats the rest)."""
+    small network a half-size batch costs 2/3 of a full one and the compaction pass eats the rest).
+
+    ``leaf_symmetry="random"``: every batch the network sees -- the whole leaf batch or a de-duplicated bucket -- is
+    first rotated / reflected row by row (oth_nn_leaf_symmetry, the orientation keyed by the engine's seed and the
+    position alone) and the network's logits are mapped back before the softmax (oth_nn_unsymmetrise_logits).
+    ``engine.nn_input`` itself is left as the step kernel wrote it."""
 
     DEDUP_BLOCK = 16  # iterations per host decision (and per throttling event)
 
-    def __init__(self, engine, evaluator=None, use_graph=True, fused=True, record=False, dedup=False):
+    def __init__(self, engine, evaluator=None, use_graph=True, fused=True, record=False, dedup=False, leaf_symmetry=None):
         """``record=True``: every launch also writes the priors / values it consumed to ``engine.priors`` /
         ``engine.values`` (fused path: what the kernel's own softmax / tanh produced), so a checker can replay them."""
+        self.leaf_symmetry = symmetry.check_mode(leaf_symmetry, ("random",))
+        if self.leaf_symmetry and engine.cfg.eval_kind != _lib.EVAL_EXTERNAL:
+            raise ValueError("leaf_symmetry needs a network evaluator: the device evaluators see no leaf planes")
         self.e = engine
         self.record = record
         # diagnostic hooks, called around every EXECUTED iteration (eager ones, the warm-up iterations of the graph
@@ -359,14 +374,34 @@ class SelfPlayRunner:
             self._events = []      # throttle: the host stays at most two blocks ahead of the device
             self._recent = [n, n]  # distinct-position counts last reported by the device
             self.bucket_iterations = {0: 0, **{b: 0 for b in self.buckets}}
+        if self.leaf_symmetry:
+            # the planes the network sees and their symmetry ids: one persistent pair per batch size (the whole batch and
+            # every bucket), so that the addresses captured in the CUDA graphs stay valid
+            sizes = [engine.n_slots] + (self.buckets if self.dedup else [])
+            self._sym = {b: (torch.zeros((b, 1, 8, 8), dtype=torch.float32, device=engine.device),
+                             torch.zeros(b, dtype=torch.uint8, device=engine.device)) for b in sizes}
+
+    def _symmetrised(self, x):
+        """(the planes the network is shown for the leaf batch ``x``, their symmetry ids or None)."""
+        if not self.leaf_symmetry:
+            return x, None
+        xs, sym = self._sym[x.size(0)]
+        symmetry.leaf_symmetry(x, self.e.cfg.seed, xs, sym)
+        return xs, sym
 
     def _iteration(self):
+        x, sym = self._symmetrised(self.e.nn_input)
         if self.external and self.fused:
-            logits, v = self.evaluator.raw(self.e.nn_input)
+            logits, v = self.evaluator.raw(x)
+            if sym is not None:
+                symmetry.unsymmetrise_logits(logits, sym)
             self.e.step_fused(logits, v, record=self.record)
             return
         if self.external:
-            self.evaluator(self.e.nn_input, self.e.priors, self.e.values)
+            if sym is None:
+                self.evaluator(x, self.e.priors, self.e.values)
+            else:
+                self.evaluator(x, self.e.priors, self.e.values, sym)
         self.e.step()
 
     def _dedup_iteration(self, bucket):
@@ -381,7 +416,10 @@ class SelfPlayRunner:
         x = self._compact[bucket]
         e.dedup(bucket, x, self._map, self._stats, self._ws)
         self._stats_host.copy_(self._stats, non_blocking=True)
+        x, sym = self._symmetrised(x)
         logits, v = self.evaluator.raw(x)
+        if sym is not None:
+            symmetry.unsymmetrise_logits(logits, sym)
         e.step_fused(logits, v, record=self.record, eval_map=self._map)
 
     def warm_start(self):

@@ -11,7 +11,7 @@ use one logged uniform per match and ply (``np.random.random_sample``), so a mat
 import numpy as np
 import torch
 
-from . import _lib, alphabeta
+from . import _lib, alphabeta, symmetry
 from .alphabeta import AlphaBetaPlayer
 from .engine import MctsEngine, private_copy
 from .envs.othello import OthelloGameNew
@@ -38,7 +38,7 @@ class DeviceStubPolicy:
 class _Side:
     """One network + one manual-mode engine holding a tree per match."""
 
-    def __init__(self, policy, args, n, device, lanes, dtype):
+    def __init__(self, policy, args, n, device, lanes, dtype, leaf_symmetry=None, seed=0):
         from .Models import fold_for_inference
         self.stub = isinstance(policy, DeviceStubPolicy)
         self.eng = MctsEngine(n, args, self_play=False, eval_kind=policy.eval_kind if self.stub else _lib.EVAL_EXTERNAL,
@@ -46,14 +46,33 @@ class _Side:
         if not self.stub:
             net = private_copy(policy, device)
             self.net = fold_for_inference(net, dtype) if dtype is not None else net
+        # a device stub sees no leaf planes: it ignores the mode
+        self.leaf_symmetry, self.seed = (None if self.stub else leaf_symmetry), int(seed)
+        if self.leaf_symmetry == "random":
+            self._xs = torch.zeros_like(self.eng.nn_input)
+            self._sym = torch.zeros(n, dtype=torch.uint8, device=self.eng.device)
+        elif self.leaf_symmetry == "mean":
+            self._images = torch.zeros((8 * n, 1, 8, 8), dtype=torch.float32, device=self.eng.device)
         self.has_tree = np.zeros(n, bool)  # "self.root is None" of the reference until the first own search
         self.record = None
 
     @torch.no_grad()
     def evaluate(self):
         e = self.eng
-        logits, value = self.net(e.nn_input)
-        torch.softmax(logits.float(), dim=-1, out=e.priors)
+        if self.leaf_symmetry == "mean":  # all eight orientations of every leaf, priors and values averaged over them
+            symmetry.images(e.nn_input, self._images)
+            logits, value = self.net(self._images)
+            symmetry.mean(logits.float(), value.float().reshape(-1), e.priors, e.values)
+            return
+        x = e.nn_input
+        if self.leaf_symmetry == "random":
+            symmetry.leaf_symmetry(x, self.seed, self._xs, self._sym)
+            x = self._xs
+        logits, value = self.net(x)
+        logits = logits.float()
+        if self.leaf_symmetry == "random":
+            symmetry.unsymmetrise_logits(logits, self._sym)
+        torch.softmax(logits, dim=-1, out=e.priors)
         e.values.copy_(value.float().reshape(-1))
 
     def search(self, mask_np, states, players, sims):
@@ -102,23 +121,28 @@ class _AlphaBetaSide:
         return alphabeta.pick(self.values[i], self.player.margin, u)
 
 
-def _side(policy, args, n, device, lanes, dtype):
-    return _AlphaBetaSide(policy, n, device) if isinstance(policy, AlphaBetaPlayer) else _Side(policy, args, n, device, lanes, dtype)
+def _side(policy, args, n, device, lanes, dtype, leaf_symmetry, seed):
+    if isinstance(policy, AlphaBetaPlayer):
+        return _AlphaBetaSide(policy, n, device)
+    return _Side(policy, args, n, device, lanes, dtype, leaf_symmetry, seed)
 
 
 def play_matches_batched(policy_a, policy_b, args, n_matches, *, device="cuda:0", lanes=None, dtype=torch.bfloat16, record=None,
-                         max_plies=128, u_tie=None):
+                         max_plies=128, u_tie=None, leaf_symmetry=None, seed=0):
     """n_matches concurrent games; match i: policy_a plays +1 if i is even, policy_b otherwise
     (eval.py:115-126).  Either policy, or both, may be a network, a ``DeviceStubPolicy`` or an ``AlphaBetaPlayer``.
     Returns (results, log): results[i] in {"A", "B", "Draw"} from policy_a's
     point of view as evaluate_models_parallel counts them; log holds per-match actions and tie uniforms.
     ``u_tie`` float64 [n_matches, max_plies]: the tie-pick uniforms to use instead of drawing them (replay of a
-    logged match, or of a match of the reference whose np.random.choice(best_actions) picks were tapped)."""
+    logged match, or of a match of the reference whose np.random.choice(best_actions) picks were tapped).
+    ``leaf_symmetry`` (network sides only): ``"random"`` shows the network every leaf in one of its eight orientations,
+    drawn from (``seed``, position); ``"mean"`` in all eight, priors and values averaged (eight network rows per leaf)."""
+    symmetry.check_mode(leaf_symmetry)
     env = OthelloGameNew(8)
     n = int(n_matches)
     sims = int(args["num_simulations"])
-    A = _side(policy_a, args, n, device, lanes, dtype)
-    B = _side(policy_b, args, n, device, lanes, dtype)
+    A = _side(policy_a, args, n, device, lanes, dtype, leaf_symmetry, seed)
+    B = _side(policy_b, args, n, device, lanes, dtype, leaf_symmetry, seed)
     A.record = B.record = record
     a_first = (np.arange(n) % 2 == 0)
     states = np.repeat(env.get_initial_state()[None], n, 0)

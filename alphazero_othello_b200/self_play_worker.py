@@ -12,7 +12,7 @@
 import numpy as np
 import torch
 
-from . import _lib, endgame
+from . import _lib, endgame, symmetry
 from .MCTS_model import MCTS
 from .engine import BatchedPolicy, MctsEngine, SelfPlayRunner, private_copy, split_games
 from .envs.othello import OthelloGameNew as OthelloGame
@@ -75,11 +75,14 @@ def one_self_play(args_tuple):
 
 
 def collect_self_play_games(policy, args, n_games, *, n_slots=None, device="cuda:0", dtype=torch.bfloat16, seed=0,
-                            game_id_base=0, fold=True, use_graph=True, return_raw=False, dedup="auto", solve_empties=0):
+                            game_id_base=0, fold=True, use_graph=True, return_raw=False, dedup="auto", solve_empties=0,
+                            leaf_symmetry=None):
     """Play ``n_games`` self-play games with ``policy`` (a torch module) on one GPU.  With ``solve_empties`` > 0 the
     value target of every position with at most that many empty squares is its solved win / draw / loss
-    (``endgame.relabel``) instead of its lambda-return."""
+    (``endgame.relabel``) instead of its lambda-return.  ``leaf_symmetry="random"``: the network sees every leaf in
+    one of its eight orientations, drawn from (``seed``, position) (``engine.SelfPlayRunner``)."""
     from .Models import fold_for_inference
+    symmetry.check_mode(leaf_symmetry, ("random",))
     if not 0 <= int(solve_empties) <= endgame.MAX_EMPTIES:
         raise ValueError(f"solve_empties must be in 0..{endgame.MAX_EMPTIES}, got {solve_empties}")
     n_slots = int(n_slots or min(n_games, 4096))
@@ -92,18 +95,20 @@ def collect_self_play_games(policy, args, n_games, *, n_slots=None, device="cuda
         ev = BatchedPolicy(net, device, torch.float32)
     else:
         ev = BatchedPolicy(net, device, dtype)
-    out = SelfPlayRunner(eng, ev, use_graph=use_graph, dedup=dedup).play()
+    out = SelfPlayRunner(eng, ev, use_graph=use_graph, dedup=dedup, leaf_symmetry=leaf_symmetry).play()
     eng.raise_on_error()
     if solve_empties:
         out = endgame.relabel(out, solve_empties, device=device)
     return out if return_raw else split_games(out)[:n_games]
 
 
-def collect_self_play_games_distributed(policy, args, n_games_per_rank, *, n_slots=None, dtype=torch.bfloat16, seed=0, version=0):
+def collect_self_play_games_distributed(policy, args, n_games_per_rank, *, n_slots=None, dtype=torch.bfloat16, seed=0, version=0,
+                                        leaf_symmetry=None):
     """Sharded ``collect_self_play_games`` (launch with torchrun, one process per GPU, NCCL initialised):
     rank 0's weights are broadcast, every rank plays its own game ids with no collective on the
     search path, and the replay tuples are gathered to rank 0, which gets the per-game lists
     (other ranks get None).  BASELINE config C5 is this with 16 384 slots per rank on 8 GPUs."""
+    symmetry.check_mode(leaf_symmetry, ("random",))
     import torch.distributed as dist
     from . import parallel
     from .Models import fold_for_inference
@@ -116,7 +121,8 @@ def collect_self_play_games_distributed(policy, args, n_games_per_rank, *, n_slo
     base, stride = parallel.shard_game_ids(rank, world, n_slots)
     eng = MctsEngine(n_slots, args, self_play=True, eval_kind=_lib.EVAL_EXTERNAL, games_per_slot=gps, device=dev, seed=seed,
                      game_id_base=base, game_id_stride=stride)
-    out = SelfPlayRunner(eng, BatchedPolicy(fold_for_inference(net, dtype), dev, torch.float32), dedup="auto").play()
+    out = SelfPlayRunner(eng, BatchedPolicy(fold_for_inference(net, dtype), dev, torch.float32), dedup="auto",
+                         leaf_symmetry=leaf_symmetry).play()
     eng.raise_on_error()
     merged = parallel.gather_replay({k: v.to(dev) for k, v in out.items() if k != "states"}, dst=0, device=dev)
     if merged is None:

@@ -429,6 +429,34 @@ int oth_nn_bias_add_relu_bf16(void* x, const void* res, const void* bias, int64_
  * stem runs as one GEMM with a fused bias+ReLU epilogue and writes channels-last output. */
 int oth_nn_stem_im2col_bf16(const float* planes, void* cols, int64_t n, void* stream);
 
+/* Network boundary: leaf symmetry.  Othello's value and move probabilities are invariant under the eight symmetries
+ * of the square; a network only approximates that.  These kernels show it a leaf in another orientation and map
+ * its outputs back.  T_s, s = 0..7, is oth_symmetry's mapping with k = s & 3 quarter turns (np.rot90) and
+ * flip = s >> 2 (np.fliplr): image[e] = plane[src_s(e)] for the 64 squares.
+ *
+ * The symmetry id of a canonical plane (+1 = side to move, -1 = opponent, as oth_mcts_step writes nn_input) is
+ *   s = philox4x32_10(seed ^ OTH_SYM_SALT; counter (own, lo32(opp), hi32(opp))).x & 7
+ * with own / opp the bitboards of the +1 / -1 squares: it depends on (seed, position) only, not on the batch row,
+ * the launch or a de-duplicated bucket, so a search's results do not depend on how its leaves were batched.
+ *
+ * oth_nn_leaf_symmetry: out_planes[i] = T_{s_i}(planes[i]) (float32 [n,64], out of place) and out_sym[i] = s_i.
+ * oth_nn_unsymmetrise_logits: in place, for the 64 square entries of each of n rows (row stride in elements, >= 65;
+ *   float32, or bfloat16 when is_bf16): row[src_s(e)] = row[e], so T_s of the result is the row the network gave.
+ *   Entry 64 (pass) and padding columns are untouched.  Softmax commutes with it: unsymmetrising the logits gives
+ *   the priors of unsymmetrising after the softmax.
+ * oth_nn_symmetry_images: out[i][j] = T_j(planes[i]), float32 [n,8,64].
+ * oth_nn_symmetry_mean: rows 8i+j (j = 0..7) of logits (float32, row stride >= 65) and values (float32, stride >= 1)
+ *   are the network's logits and tanh'd value for image j of leaf i; priors[i] (float32 [n,65]) =
+ *   (1/8) sum_j unsym_j(softmax(logits[8i+j])) and out_values[i] = (1/8) sum_j values[8i+j], summed in the
+ *   order j = 0..7.
+ * Bad sizes, strides, NULL or misaligned pointers return OTH_E_ARG before any device call; n = 0 is a no-op. */
+#define OTH_SYM_SALT 0x73796D6D65747279ull /* "symmetry" */
+int oth_nn_leaf_symmetry(const float* planes, int64_t n, uint64_t seed, float* out_planes, uint8_t* out_sym, void* stream);
+int oth_nn_unsymmetrise_logits(void* logits, int64_t stride, int32_t is_bf16, const uint8_t* sym, int64_t n, void* stream);
+int oth_nn_symmetry_images(const float* planes, int64_t n, float* out, void* stream);
+int oth_nn_symmetry_mean(const float* logits, int64_t stride, const float* values, int64_t value_stride, int64_t n,
+                         float* priors, float* out_values, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
